@@ -4,7 +4,7 @@ chunks (BASELINE.json configs[1]) at N GPUs, with the HBM roofline fraction of t
 kernel and the reference's CPU path timed beside it; the other BASELINE configs ride along in a
 `secondary` array of the same JSON line.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 One "step" = one pass of the FIR over one 64 Mi-sample chunk per GPU, taken from a device-resident
@@ -261,6 +261,24 @@ def _time_passes(torch, fn, reps, warm=1):
     e[1].record()
     torch.cuda.synchronize()
     return e[0].elapsed_time(e[1]) * 1e-3 / reps
+
+
+DUMP_HEAD = 4096                  # --dump-outputs keeps the first outputs (their window reaches into the history) ...
+DUMP_SAMPLES = 1 << 20            # ... and a seeded sample of the rest: 8 MiB of values, 8 MiB of indices
+
+
+def dump_outputs(path, out, consumed, produced, status):
+    """Writes what the last timed step returned to its caller, so that two builds can be compared output for output:
+    fir_counts.npy = (consumed, produced, status), fir_out.npy = (re, im) float32 of the outputs at fir_out_index.npy.
+    The indices are the same in every run (all 64 Mi outputs would be 512 MiB)."""
+    import torch
+    os.makedirs(path, exist_ok=True)
+    pick = np.random.default_rng(SEED).choice(produced, size=min(produced, DUMP_SAMPLES), replace=False)
+    idx = np.union1d(np.arange(min(produced, DUMP_HEAD)), pick)
+    vals = torch.view_as_real(out[:produced].index_select(0, torch.from_numpy(idx).to(out.device)))
+    np.save(os.path.join(path, "fir_counts.npy"), np.array([consumed, produced, int(status)], np.float64))
+    np.save(os.path.join(path, "fir_out_index.npy"), idx.astype(np.float64))
+    np.save(os.path.join(path, "fir_out.npy"), vals.cpu().numpy())
 
 
 def _roofline(alg_bytes, sec, note=None):
@@ -882,6 +900,8 @@ def run_ours(args):
         print(f"host_step rank {rank}: {host_step_us:.1f} us to enqueue one step", file=sys.stderr, flush=True)
     barrier()
     launches = ctx.launch_count - l0
+    if args.dump_outputs and rank == 0:          # before the sustained run below overwrites `out`
+        dump_outputs(args.dump_outputs, out, c, p, st)
     clocks = sampler.stop() if rank == 0 else None
     total_ms = ev[0].elapsed_time(ev[-1])
     kern_ms = [a.elapsed_time(b) for a, b in kev]
@@ -1066,7 +1086,13 @@ def main():
     ap.add_argument("--no-sustained", action="store_true", help="skip the >= 1 s sustained run")
     ap.add_argument("--exchange", default="peer", choices=["peer", "nccl", "none"],
                     help="halo exchange of the sharded stream: in-kernel peer fetch over NVLink (default) or NCCL all-gather")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the last step's results (rank 0) to DIR as .npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs records the device path (--impl ours)")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.impl == "reference":
         run_reference(args)
